@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — VirConv-L backbone scenes/s (forward+backward) on synthetic KITTI-shaped scenes.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" = one forward+backward pass of the VirConv-L 3-D backbone (20 sparse convs + BN/ReLU + 4x index2uv,
@@ -14,6 +14,12 @@ reference grid [81,1600,1408]).  One JSON line on rank 0 (contract: task stateme
   roofline  the dominant kernel (gather-GEMM: conv forward + dgrad launches): algorithmic bytes / event time
   cpu_baseline / --impl reference : the restated reference algorithm (spconv "Native": CPU hash-map rulebook +
             per-offset torch.mm + index_add_) from oracle/, timed on this box's host cores.
+
+--dump-outputs DIR writes what the last timed step of `value` computed, as a caller of the step receives it: the loss
+(DIR/loss.npy) and every parameter gradient (DIR/grad.<parameter name>.npy), float32.  Inputs and initial weights are
+seeded, so two builds run with the same arguments can be compared output for output.  The gradients are accumulated
+with float atomics, so two runs of one build already differ slightly (bf16, on a B200 at 1000 W: loss bit-identical,
+gradients up to 3.4e-3 of a tensor's largest element apart).
 """
 from __future__ import annotations
 
@@ -61,7 +67,7 @@ class _StdoutToStderr:
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20, help='timed steps per measurement (at least 1)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
@@ -89,7 +95,24 @@ def parse():
                     help='graph mode: 1 = graph.PipelinedStep (index graph of step t+1 beside the feature graph of step t), 0 = one graph per step')
     ap.add_argument('--ncu-step', action='store_true',
                     help='profiling aid: W warm-up steps, then exactly one step between cudaProfilerStart/Stop; no JSON')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='VirConv-L: write the loss and parameter gradients of the last timed step as DIR/<name>.npy')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and (a.impl != 'ours' or a.model != 'L' or a.ncu_step):
+        ap.error('--dump-outputs applies to the VirConv-L measurement of --impl ours')
+    return a
+
+
+def dump_outputs(out_dir, loss, named_params):
+    """The step's outputs as float32 .npy files: loss.npy and grad.<parameter name>.npy (zeros for a parameter the loss
+    does not reach)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'loss.npy'), loss.detach().float().reshape(1).cpu().numpy())
+    for name, p in named_params:
+        g = p.grad if p.grad is not None else torch.zeros_like(p)
+        np.save(os.path.join(out_dir, f'grad.{name}.npy'), g.detach().float().cpu().numpy())
 
 
 def peaks():
@@ -530,6 +553,7 @@ def run_ours(args):
     copy_stream = torch.cuda.Stream(device=dev)
     main_stream = torch.cuda.current_stream(dev)
     loss_host = torch.zeros(4096, dtype=torch.float32).pin_memory()
+    last_loss = [None]
 
     def timed(n_steps, from_host):
         """from_host (the e2e loop): every step uploads its inputs from PINNED host memory and reads its loss back into
@@ -561,9 +585,10 @@ def run_ours(args):
             else:
                 vf, vc, b = devb[s % POOL]
                 if graphed is not None:
-                    gstep(*dev_p[s % POOL])
+                    loss = gstep(*dev_p[s % POOL])
                 else:
-                    step(vf, vc, b, False, resident=True)
+                    loss = step(vf, vc, b, False, resident=True)
+            last_loss[0] = loss
             e.record()
             evs.append((a, e))
         torch.cuda.synchronize()
@@ -604,6 +629,9 @@ def run_ours(args):
     if graphed is not None:
         launches = graphed.launches_per_replay        # kernels of this library inside the captured step (counted at capture)
     dev_allocs = torch.cuda.memory_stats(dev).get('num_device_alloc', 0) - dev_allocs0
+    if args.dump_outputs and rank == 0:
+        # before anything else runs a step: the graph's loss and the .grad tensors are rewritten by every step
+        dump_outputs(args.dump_outputs, last_loss[0], model.named_parameters())
     timed(max(2, min(args.steps, 10)), True)      # warm-up + allocator priming of the e2e loop
     barrier()
     st0 = torch.cuda.memory_stats(dev)

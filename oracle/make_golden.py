@@ -9,9 +9,12 @@ What the reference can pin (it ships no tests and no spconv):
     strides handed to index2uv, published outputs), executed by the reference's classes with the
     ORACLE's CPU sparse-conv operators standing in for the absent spconv package
                                                                          -> golden/virconv_l_small.npz
+  * the StVD input point discard of `DatasetTemplate`                   -> golden/stvd_input.npz
+  * the backbones' state_dict layout over spconv_compat (own process)    -> golden/reference_backbones.json
+  * the stacked pointnet2 CUDA kernels, built into oracle/_ref (on a GPU) -> golden/roi_pool.npz
 The sparse-conv arithmetic itself stays pinned only by the dense-conv property tests.
 
-usage:  python -m oracle.make_golden
+usage:  python -m oracle.make_golden [main | backbone_layout | roi_pool]
 """
 from __future__ import annotations
 
@@ -101,21 +104,120 @@ def stvd_golden():
         same = ref.shape == mine.shape and np.array_equal(ref, mine, equal_nan=True)
         report.append(f'StVD input discard {name}: N={pts.shape[0]} -> {ref.shape[0]} rows, restated == reference: {same}')
         assert same, name
-        out[f'{name}:points'] = pts
-        out[f'{name}:out'] = ref
+        # the output rows are rows of the input cloud: stored as their row numbers, every cloud once
+        cloud = name.split('_bins')[0]
+        assert np.array_equal(out.setdefault(f'{cloud}:points', pts), pts, equal_nan=True), name
+        row_of = {r.tobytes(): i for i, r in reversed(list(enumerate(pts)))}
+        out[f'{name}:cloud'] = np.array(cloud)
+        out[f'{name}:out_rows'] = np.array([row_of[r.tobytes()] for r in ref], dtype=np.int32).reshape(-1)
+        assert np.array_equal(pts[out[f'{name}:out_rows']], ref, equal_nan=True), name
         out[f'{name}:meta'] = np.array([bn, seed], dtype=np.int64)
         out[f'{name}:rate'] = np.float64(rate)
     np.savez_compressed(os.path.join(OUT, 'stvd_input.npz'), **out)
     return report
 
 
+def backbone_layout_golden():
+    """tests/golden/reference_backbones.json: the reference's VirConvL8x / VirConv8x classes (spconv_backbone.py)
+    constructed over `spconv_compat.install_as_spconv()` — state_dict entries in order as 'key (shape) dtype',
+    num_point_features, sparse_shape and, per sparse convolution in module order, whether it has a bias."""
+    import json
+    from virconv_b200 import spconv_compat
+    spconv_compat.install_as_spconv()
+    for name, rel in [('pcdet', 'pcdet'), ('pcdet.utils', 'pcdet/utils'), ('pcdet.datasets', 'pcdet/datasets'),
+                      ('pcdet.datasets.augmentor', 'pcdet/datasets/augmentor'), ('pcdet.models', 'pcdet/models'),
+                      ('pcdet.models.backbones_3d', 'pcdet/models/backbones_3d')]:
+        pkg = types.ModuleType(name)
+        pkg.__path__ = [os.path.join(REF, rel)]
+        sys.modules[name] = pkg
+    for stub in ('pcdet.utils.box_utils', 'pcdet.utils.box_np_ops'):
+        sys.modules[stub] = types.ModuleType(stub)
+    bb = importlib.import_module('pcdet.models.backbones_3d.spconv_backbone')
+    assert bb.spconv is spconv_compat
+    cfgs = {'VirConvL8x': AttrDict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.1,
+                                   NUM_FILTERS=[16, 32, 64, 64]),
+            'VirConv8x': AttrDict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.15,
+                                  NUM_FILTERS=[16, 32, 64, 64], MM=True)}
+    out = {}
+    for name, cfg in cfgs.items():
+        r = getattr(bb, name)(model_cfg=cfg, input_channels=8, grid_size=np.array([1408, 1600, 80]))
+        out[name] = {'state_dict': [f'{k} {tuple(v.shape)} {v.dtype}' for k, v in r.state_dict().items()],
+                     'num_point_features': r.num_point_features, 'sparse_shape': [int(s) for s in r.sparse_shape],
+                     'conv_has_bias': [m.bias is not None for m in r.modules()
+                                       if isinstance(m, spconv_compat.SparseConvolution)]}
+    path = os.path.join(OUT, 'reference_backbones.json')
+    with open(path, 'w') as f:
+        json.dump(out, f, indent=1)
+        f.write('\n')
+    return path
+
+
+def roi_pool_golden():
+    """tests/golden/roi_pool.npz: the reference's own stacked pointnet2 kernels (oracle/_ref, oracle/ref_build.py) on the
+    full-size cases of oracle/pointnet2.py — voxel query, grouping of features and of xyz, grouping gradient.  Needs a GPU.
+    Stored per case: the empty-ball mask, seeded row samples of every output, the largest gradient magnitude, and SHA-256
+    digests of the complete index and grouping outputs (both are exact: integer indices and pure gathers)."""
+    import ctypes
+    from . import pointnet2 as o_pn
+    from . import ref_build
+    from .testing import sha256_bytes as sha256
+    lib = ctypes.CDLL(ref_build.build())
+    p = lambda t: ctypes.c_void_p(t.data_ptr())
+    d = lambda a: torch.from_numpy(a).cuda()
+    xyz, xyz_cnt, new_xyz, new_cnt, new_coords, v2p = o_pn.scene(1)
+    M, N, C = new_coords.shape[0], xyz.shape[0], o_pn.ROI_CHANNELS
+    t_xyz, t_new_xyz, t_coords, t_v2p, cnt_f, cnt_q = d(xyz), d(new_xyz), d(new_coords), d(v2p), d(xyz_cnt), d(new_cnt)
+    starts = np.concatenate([[0], np.cumsum(xyz_cnt)[:-1]]).astype(np.int32)
+    out = {}
+    for ci, (max_range, radius, nsample) in enumerate(o_pn.ROI_CASES):
+        key = o_pn.roi_case_key(max_range, radius, nsample)
+        feats, grad_out = o_pn.roi_case_data(max_range, radius, nsample, N, M)
+        # the kernel + the two lines of VoxelQuery.forward around it (voxel_query_utils.py:32-39)
+        ridx = torch.zeros((M, nsample), dtype=torch.int32, device='cuda')
+        torch.cuda.synchronize()
+        lib.ref_voxel_query(M, v2p.shape[1], v2p.shape[2], v2p.shape[3], nsample, ctypes.c_float(radius), *max_range,
+                            p(t_new_xyz), p(t_xyz), p(t_coords), p(t_v2p), p(ridx))
+        torch.cuda.synchronize()
+        empty = ridx[:, 0] == -1
+        ridx[empty] = 0
+        # grouping forward / backward as VoxelQueryAndGrouping.forward (:80-99) calls it: batch-local indices
+        lidx = (ridx.view(len(xyz_cnt), -1, nsample) - d(starts).view(-1, 1, 1)).view(-1, nsample)
+        lidx[empty] = 0
+        lidx = lidx.contiguous()
+        fc, go = d(feats), d(grad_out)
+        rgf = torch.empty((M, C, nsample), device='cuda')
+        rgx = torch.empty((M, 3, nsample), device='cuda')
+        rg = torch.zeros((N, C), device='cuda')
+        torch.cuda.synchronize()
+        lib.ref_group_points(len(xyz_cnt), M, C, nsample, p(fc), p(cnt_f), p(lidx), p(cnt_q), p(rgf))
+        lib.ref_group_points(len(xyz_cnt), M, 3, nsample, p(t_xyz), p(cnt_f), p(lidx), p(cnt_q), p(rgx))
+        lib.ref_group_points_grad(len(xyz_cnt), M, C, N, nsample, p(go), p(lidx), p(cnt_q), p(cnt_f), p(rg))
+        torch.cuda.synchronize()
+        ridx, empty, rgf, rgx, rg = (t.cpu().numpy() for t in (ridx, empty, rgf, rgx, rg))
+        rng = np.random.default_rng(300 + ci)
+        idx_rows = np.sort(rng.choice(M, 256, replace=False))
+        group_rows = np.sort(rng.choice(M, 8, replace=False))
+        # row 0 of every sample collects the gradient of all empty balls: always in the sample
+        grad_rows = np.union1d(starts, rng.choice(N, 128, replace=False))
+        out.update({f'{key}:empty': np.packbits(empty), f'{key}:idx_rows': idx_rows, f'{key}:idx': ridx[idx_rows],
+                    f'{key}:idx_sha256': np.array(sha256(ridx)), f'{key}:group_rows': group_rows,
+                    f'{key}:features': rgf[group_rows], f'{key}:features_sha256': np.array(sha256(rgf)),
+                    f'{key}:xyz': rgx[group_rows], f'{key}:xyz_sha256': np.array(sha256(rgx)),
+                    f'{key}:grad_rows': grad_rows, f'{key}:grad': rg[grad_rows],
+                    f'{key}:grad_absmax': np.float32(np.abs(rg).max())})
+    path = os.path.join(OUT, 'roi_pool.npz')
+    np.savez_compressed(path, **out)
+    return path
+
+
 def main():
     from virconv_b200 import scenes
     from . import index2uv as o_uv
-    from .testing import fill_module
+    from .testing import GOLDEN_THREADS, fill_module, sampled_rows
     from .backbone import VirConvL8x as OracleL
 
     bb, calib_mod, vfe_mod = import_reference()
+    torch.set_num_threads(GOLDEN_THREADS)
     os.makedirs(OUT, exist_ok=True)
     calib_dict = {'P2': scenes.P2, 'R0': scenes.R0, 'Tr_velo2cam': scenes.TR_VELO_TO_CAM}
     report = []
@@ -208,7 +310,7 @@ def main():
                 err = float((t.features - o[k].features).abs().max() / t.features.abs().max())
                 lines.append(f'VirConvL8x[{mode}] {k}: N={t.features.shape[0]} C={t.features.shape[1]} '
                              f'indices identical={same_idx} rel err restated-vs-reference-flow={err:.2e}')
-                out[f'{mode}_{k}_features'] = t.features.numpy()
+                out.update(sampled_rows(f'{mode}_{k}_features', t.features.numpy()))
                 out[f'{mode}_{k}_indices'] = t.indices.numpy().astype(np.int32)
         if flips == 0:
             report.append(f'VirConvL8x fixture: scenes ({first_scene},{first_scene + 1}), no pixel-cell flips')
@@ -257,10 +359,10 @@ def main():
                     same &= np.array_equal(t.indices.numpy(), rt.indices.numpy())
                     if same:
                         worst = max(worst, float((t.features - rt.features).abs().max() / rt.features.abs().max().clamp_min(1e-30)))
-                    tensors[f'{mode}:{key}:{name}:features'] = rt.features.numpy()
+                    tensors.update(sampled_rows(f'{mode}:{key}:{name}:features', rt.features.numpy()))
                     tensors[f'{mode}:{key}:{name}:indices'] = rt.indices.numpy().astype(np.int32)
             if same and worst == 0.0:
-                report.append(f'VirConv8x[{mode}] fixture: scenes ({first_scene},{first_scene + 1}), {len(tensors) // 2} published '
+                report.append(f'VirConv8x[{mode}] fixture: scenes ({first_scene},{first_scene + 1}), {len(tensors) // 5} published '
                               f'tensors, indices identical, restated-vs-reference-flow rel err 0')
                 gold8.update(tensors)
                 for k, v in bm.arrays.items():
@@ -280,4 +382,5 @@ def main():
 
 
 if __name__ == '__main__':
-    main()
+    what = sys.argv[1] if len(sys.argv) > 1 else 'main'
+    print({'main': main, 'backbone_layout': backbone_layout_golden, 'roi_pool': roi_pool_golden}[what]())

@@ -76,3 +76,15 @@ def input_point_discard(points, bin_num=2, rate=0.8, rng=np.random):
             rands = rng.permutation(parts[i].shape[0])
             parts[i] = parts[i][rands[:per_bin]]
     return np.concatenate(parts)
+
+
+def golden_cases(g):
+    """The cases of tests/golden/stvd_input.npz (oracle/make_golden.py): each input cloud is stored once
+    ('<cloud>:points'), each case names its cloud ('<case>:cloud') and gives its output as rows of it ('<case>:out_rows').
+    -> [(case name, points, bin_num, rate, seed, expected output)]"""
+    out = []
+    for name in sorted(k[:-len(':cloud')] for k in g.files if k.endswith(':cloud')):
+        pts = g[f'{g[name + ":cloud"]}:points']
+        bn, seed = (int(v) for v in g[f'{name}:meta'])
+        out.append((name, pts, bn, float(g[f'{name}:rate']), seed, pts[g[f'{name}:out_rows']]))
+    return out

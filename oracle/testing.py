@@ -1,6 +1,10 @@
-"""Deterministic parameter filling shared by the golden-vector script and the tests.
+"""Deterministic parameter filling and the compact golden-array format, shared by the golden-vector script and the tests.
 TEST INFRASTRUCTURE (see oracle/__init__.py)."""
 from __future__ import annotations
+
+import contextlib
+import hashlib
+import zlib
 
 import numpy as np
 import torch
@@ -39,6 +43,54 @@ def rel_err(got, want):
     got = torch.as_tensor(got).double()
     want = torch.as_tensor(want).double()
     return float((got - want).abs().max() / want.abs().max().clamp_min(1e-30))
+
+
+# Train-mode BatchNorm on the CPU sums its batch statistics in per-thread partial sums, so the last bits of its output
+# follow torch's intra-op thread count; the bit-exact fixtures of tests/golden/ are made and checked with this many threads.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
+
+
+def sha256_bytes(a) -> str:
+    """SHA-256 of an array's (or tensor's) bytes in C order."""
+    return hashlib.sha256(np.ascontiguousarray(torch.as_tensor(a).detach().cpu().numpy()).tobytes()).hexdigest()
+
+
+def sha256_f32(a) -> str:
+    """SHA-256 of an array as float32 bytes, -0.0 folded into +0.0 (np.array_equal's notion of equal, NaN aside)."""
+    return sha256_bytes(np.asarray(torch.as_tensor(a).detach().cpu().numpy(), dtype=np.float32) + np.float32(0))
+
+
+def sampled_rows(key, a):
+    """A golden float array stored compactly: a seeded quarter of its rows (`key`, row numbers in `key.rows`) plus what a
+    comparison of the whole array needs — its digest (`key.sha256`) and its largest magnitude (`key.absmax`)."""
+    a = np.asarray(a, dtype=np.float32)
+    rng = np.random.default_rng(zlib.crc32(key.encode()))
+    rows = np.sort(rng.choice(a.shape[0], -(-a.shape[0] // 4), replace=False)).astype(np.int32)
+    return {key: a[rows], key + '.rows': rows, key + '.sha256': np.array(sha256_f32(a)),
+            key + '.absmax': np.float32(np.abs(a).max() if a.size else 0)}
+
+
+def check_sampled_rows(got, g, key, tol=None):
+    """`got` against an array stored by sampled_rows in the npz `g`.  tol None: bit-exact — the sampled rows, then the
+    digest of the whole array.  Otherwise rel_err on the sampled rows, relative to the whole golden array's max |x|."""
+    got = torch.as_tensor(got).detach().cpu()
+    rows = torch.from_numpy(g[key + '.rows']).long()
+    if tol is None:
+        assert np.array_equal(got[rows].numpy(), g[key]), key
+        assert sha256_f32(got) == str(g[key + '.sha256']), key
+    else:
+        err = float((got[rows].double() - torch.from_numpy(g[key]).double()).abs().max()) if len(rows) else 0.0
+        assert err / max(float(g[key + '.absmax']), 1e-30) < tol, (key, err)
 
 
 def join_by_coords(idx_a, feat_a, idx_b, feat_b):

@@ -11,7 +11,7 @@ from oracle import index2uv as ouv
 from oracle import rulebook as orb
 from oracle import spconv_cpu as osp
 from oracle.backbone import VirConvL8x as OracleL
-from oracle.testing import fill_module, rel_err
+from oracle.testing import check_sampled_rows, fill_module, golden_threads, rel_err
 from virconv_b200 import scenes
 
 GOLD = os.path.join(os.path.dirname(__file__), 'golden')
@@ -70,12 +70,12 @@ def test_oracle_backbone_matches_reference_flow_golden(mode):
     m = OracleL()
     fill_module(m, int(g['seed']))
     m.train(mode == 'train')
-    with torch.no_grad():
+    with torch.no_grad(), golden_threads():
         o = m(torch.from_numpy(g['voxel_features'].copy()), torch.from_numpy(g['voxel_coords'].copy()), 2,
               [scenes.Calib(), scenes.Calib()], g['aug_param'])
     for k in ('x_conv1', 'x_conv2', 'x_conv3', 'x_conv4', 'out'):
         assert np.array_equal(o[k].indices.numpy(), g[f'{mode}_{k}_indices'])
-        assert np.array_equal(o[k].features.numpy(), g[f'{mode}_{k}_features'])
+        check_sampled_rows(o[k].features, g, f'{mode}_{k}_features')
 
 
 def test_scene_generator_is_deterministic_and_kitti_shaped():
@@ -169,7 +169,7 @@ def test_oracle_virconv8x_matches_reference_flow_golden(mode):
     m.train(mode == 'train')
     arrays = {k.split(':')[2]: torch.from_numpy(g[k].copy()) for k in g.files if k.startswith(f'{mode}:in:')}
     kw = dict(aug_param=g[f'{mode}:aug']) if mode == 'train' else dict(transform_param=g[f'{mode}:aug'])
-    with torch.no_grad():
+    with torch.no_grad(), golden_threads():
         o = m(arrays, 2, [scenes.Calib(), scenes.Calib()], **kw)
     n = 0
     for k in g.files:
@@ -178,29 +178,21 @@ def test_oracle_virconv8x_matches_reference_flow_golden(mode):
             continue
         t = o[parts[1]] if parts[2] == 'out' else o[parts[1]][parts[2]]
         assert np.array_equal(t.indices.numpy(), g[f'{mode}:{parts[1]}:{parts[2]}:indices'])
-        assert np.array_equal(t.features.numpy(), g[k])
+        check_sampled_rows(t.features, g, k)
         n += 1
     assert n == (9 if mode == 'train' else 21)
 
 
 # ---------------------------------------------------------------------------------------- StVD input point discard
-def _stvd_cases():
-    g = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'stvd_input.npz'))
-    names = sorted({k.split(':')[0] for k in g.files})
-    return g, names
-
-
 def test_stvd_input_discard_oracle_matches_reference_golden():
     """tests/golden/stvd_input.npz holds outputs of the reference's OWN `DatasetTemplate.input_point_discard`
     (dataset.py:168-189) under seeded np.random (oracle/make_golden.py): the restatement must reproduce every row."""
     from oracle import stvd
-    g, names = _stvd_cases()
-    assert len(names) >= 10
-    for name in names:
-        bn, seed = (int(v) for v in g[f'{name}:meta'])
-        out = stvd.input_point_discard(g[f'{name}:points'].copy(), bin_num=bn, rate=float(g[f'{name}:rate']),
-                                       rng=np.random.RandomState(seed))
-        assert np.array_equal(out, g[f'{name}:out'], equal_nan=True), name
+    cases = stvd.golden_cases(np.load(os.path.join(GOLD, 'stvd_input.npz')))
+    assert len(cases) >= 10
+    for name, pts, bn, rate, seed, want in cases:
+        out = stvd.input_point_discard(pts.copy(), bin_num=bn, rate=rate, rng=np.random.RandomState(seed))
+        assert np.array_equal(out, want, equal_nan=True), name
 
 
 def test_stvd_host_plan_of_the_product_matches_oracle():

@@ -1,9 +1,11 @@
-"""Drop-in boundary, checked against the reference's OWN unmodified files (only where /root/reference exists, i.e. in the
-build container — the GPU box has no copy): `pcdet/models/backbones_3d/spconv_backbone.py` and the dataloader's
-`VoxelGeneratorWrapper` (`pcdet/datasets/processor/data_processor.py:13-59`) import and construct over
-`spconv_compat.install_as_spconv()` (SURVEY §8b items 1-3), and produce the state_dict keys / voxel arrays this repo's own
-classes produce."""
-import importlib
+"""Drop-in boundary against the reference's OWN unmodified files: its backbone classes
+(`pcdet/models/backbones_3d/spconv_backbone.py`) and the dataloader's `VoxelGeneratorWrapper`
+(`pcdet/datasets/processor/data_processor.py:13-59`) construct and run over `spconv_compat.install_as_spconv()`
+(SURVEY §8b items 1-3).  What the reference's classes produce over the shim is stored in
+tests/golden/reference_backbones.json (oracle/make_golden.py backbone_layout); the whole-detector build needs the
+reference's `pcdet` package itself and runs only where a copy of it is found."""
+import ast
+import json
 import os
 import sys
 import types
@@ -12,7 +14,8 @@ import numpy as np
 import pytest
 
 REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'pcdet')), reason='no /root/reference on this machine')
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'pcdet')), reason='the reference pcdet package is not present')
+GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 
 class AttrDict(dict):
@@ -34,71 +37,68 @@ def _restore_modules(saved):
 
 
 @pytest.fixture()
-def reference_pkgs():
-    """Stub package objects for pcdet (its real __init__ files import compiled ops) + this repo's spconv / cumm shims;
-    everything is removed from sys.modules again afterwards."""
+def spconv_shims():
+    """`spconv` / `cumm` resolved to this repo's shims; removed from sys.modules again afterwards."""
     saved = dict(sys.modules)
     from virconv_b200 import spconv_compat
     spconv_compat.install_as_spconv()
-    for name, rel in [('pcdet', 'pcdet'), ('pcdet.utils', 'pcdet/utils'), ('pcdet.datasets', 'pcdet/datasets'),
-                      ('pcdet.datasets.augmentor', 'pcdet/datasets/augmentor'),
-                      ('pcdet.datasets.processor', 'pcdet/datasets/processor'), ('pcdet.models', 'pcdet/models'),
-                      ('pcdet.models.backbones_3d', 'pcdet/models/backbones_3d')]:
-        pkg = types.ModuleType(name)
-        pkg.__path__ = [os.path.join(REF, rel)]
-        sys.modules[name] = pkg
-    for stub in ('pcdet.utils.box_utils', 'pcdet.utils.box_np_ops', 'skimage', 'skimage.transform'):
-        m = types.ModuleType(stub)
-        m.__path__ = []
-        sys.modules[stub] = m
-    sys.modules['skimage'].transform = sys.modules['skimage.transform']
     try:
         yield
     finally:
         _restore_modules(saved)
 
 
-def test_reference_backbones_construct_over_spconv_compat(reference_pkgs):
+def test_reference_backbones_construct_over_spconv_compat():
+    """Our classes against the reference's classes built over the shim (golden): state_dict keys in order, shapes and
+    dtypes, num_point_features, sparse_shape, bias-free sparse convolutions; a checkpoint of the reference's layout loads."""
     import torch
     from virconv_b200 import backbone as ours
     from virconv_b200 import spconv_compat
-    ref = importlib.import_module('pcdet.models.backbones_3d.spconv_backbone')
-    assert ref.spconv is spconv_compat                          # `import spconv.pytorch as spconv` resolved to the shim
-    cfg_l = AttrDict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.1, NUM_FILTERS=[16, 32, 64, 64])
-    cfg_t = AttrDict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.15, NUM_FILTERS=[16, 32, 64, 64],
-                     MM=True)
+    gold = json.load(open(os.path.join(GOLD, 'reference_backbones.json')))
+    cfg_l = dict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.1, NUM_FILTERS=[16, 32, 64, 64])
+    cfg_t = dict(RETURN_NUM_FEATURES_AS_DICT=True, OUT_FEATURES=64, LAYER_DISCARD_RATE=0.15, NUM_FILTERS=[16, 32, 64, 64],
+                 MM=True)
     for name, cfg in (('VirConvL8x', cfg_l), ('VirConv8x', cfg_t)):
-        torch.manual_seed(0)
-        r = getattr(ref, name)(model_cfg=cfg, input_channels=8, grid_size=np.array([1408, 1600, 80]))
-        o = getattr(ours, name)(dict(cfg), 8, [1408, 1600, 80])
-        rs, os_ = r.state_dict(), o.state_dict()
-        assert list(rs.keys()) == list(os_.keys()), name
-        assert all(tuple(rs[k].shape) == tuple(os_[k].shape) for k in rs), name
-        assert r.num_point_features == o.num_point_features, name
-        assert list(r.sparse_shape) == list(o.sparse_shape), name
-        # a checkpoint written by the reference class loads into ours and vice versa (weight layout (C_out, *k, C_in))
-        o.load_state_dict(rs)
-        r.load_state_dict(os_)
-        convs = [m for m in r.modules() if isinstance(m, spconv_compat.SparseConvolution)]
+        g = gold[name]
+        o = getattr(ours, name)(cfg, 8, [1408, 1600, 80])
+        os_ = o.state_dict()
+        assert [f'{k} {tuple(v.shape)} {v.dtype}' for k, v in os_.items()] == g['state_dict'], name
+        assert o.num_point_features == g['num_point_features'], name
+        assert list(o.sparse_shape) == g['sparse_shape'], name
+        # a checkpoint of the reference class's layout loads into ours (weight layout (C_out, *k, C_in))
+        ckpt = {}
+        for entry in g['state_dict']:
+            k, rest = entry.split(' ', 1)
+            shape, dtype = rest.rsplit(' ', 1)
+            ckpt[k] = torch.ones(ast.literal_eval(shape), dtype=getattr(torch, dtype.split('.')[1]))
+        o.load_state_dict(ckpt)
+        convs = [m for m in o.modules() if isinstance(m, spconv_compat.SparseConvolution)]
+        assert [m.bias is not None for m in convs] == g['conv_has_bias'], name
         assert len(convs) == (20 if name == 'VirConvL8x' else 31), (name, len(convs))
-        assert all(m.bias is None for m in convs)
 
 
-def test_reference_voxel_generator_wrapper_runs_over_the_shims(reference_pkgs):
+def test_reference_voxel_generator_wrapper_runs_over_the_shims(spconv_shims):
+    """The wrapper's spconv-2 branch over the shims: `spconv.utils` offers neither VoxelGeneratorV2 nor VoxelGenerator, so it
+    builds `Point2VoxelCPU3d(vsize_xyz=, coors_range_xyz=, num_point_features=, max_num_points_per_voxel=, max_num_voxels=)`,
+    calls `point_to_voxel(tv.from_numpy(points))` and takes `.numpy()` of the three outputs."""
     from virconv_b200 import scenes
-    dp = importlib.import_module('pcdet.datasets.processor.data_processor')
-    assert dp.tv is not None                                    # `import cumm.tensorview as tv` resolved
-    gen = dp.VoxelGeneratorWrapper(vsize_xyz=[0.05, 0.05, 0.05], coors_range_xyz=[0, -40, -3, 70.4, 40, 1], num_point_features=8,
-                                   max_num_points_per_voxel=5, max_num_voxels=4000)
-    assert gen.spconv_ver == 2
+    with pytest.raises(ImportError):
+        from spconv.utils import VoxelGeneratorV2  # noqa: F401
+    with pytest.raises(ImportError):
+        from spconv.utils import VoxelGenerator  # noqa: F401
+    from spconv.utils import Point2VoxelCPU3d
+    import cumm.tensorview as tv
+    gen = Point2VoxelCPU3d(vsize_xyz=[0.05, 0.05, 0.05], coors_range_xyz=[0, -40, -3, 70.4, 40, 1], num_point_features=8,
+                           max_num_points_per_voxel=5, max_num_voxels=4000)
     pts = scenes.make_points(3, n_lidar=2048, n_virtual=6000)
-    voxels, coords, num = gen.generate(pts)
+    voxels, coords, num = (t.numpy() for t in gen.point_to_voxel(tv.from_numpy(pts)))
     v0, c0, n0 = scenes.voxelize_first_come(pts, max_points=5, max_voxels=4000)
     assert voxels.shape == (4000, 5, 8) and coords.shape == (4000, 3) and num.shape == (4000,)
     assert np.array_equal(voxels, v0) and np.array_equal(coords, c0) and np.array_equal(num, n0)
     assert coords[:, 0].max() < 80 and coords[:, 2].max() > 80 and coords[:, 2].max() < 1408         # zyx order
 
 
+@needs_reference
 @pytest.mark.parametrize('yaml_name', ['VirConv-L.yaml', 'VirConv-T.yaml', 'VirConv-S.yaml'])
 def test_reference_detector_builds_under_reference_env(yaml_name, monkeypatch):
     """SURVEY §8f-2: with `reference_env.install()` the reference's unmodified `pcdet` package imports on this stack (py3.12,

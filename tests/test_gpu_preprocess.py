@@ -15,14 +15,10 @@ GOLD = os.path.join(os.path.dirname(__file__), 'golden')
 
 def test_stvd_input_discard_matches_reference_golden(lib_built):
     from virconv_b200 import preprocess
-    g = np.load(os.path.join(GOLD, 'stvd_input.npz'))
-    names = sorted({k.split(':')[0] for k in g.files})
-    for name in names:
-        bn, seed = (int(v) for v in g[f'{name}:meta'])
-        pts = torch.from_numpy(g[f'{name}:points'].copy()).cuda()
+    for name, pts, bn, rate, seed, want in o_stvd.golden_cases(np.load(os.path.join(GOLD, 'stvd_input.npz'))):
         np.random.seed(seed)                                            # the reference draws from the global generator
-        out = preprocess.input_point_discard(pts, bin_num=bn, rate=float(g[f'{name}:rate']))
-        assert np.array_equal(out.cpu().numpy(), g[f'{name}:out'], equal_nan=True), name
+        out = preprocess.input_point_discard(torch.from_numpy(pts.copy()).cuda(), bin_num=bn, rate=rate)
+        assert np.array_equal(out.cpu().numpy(), want, equal_nan=True), name
 
 
 @pytest.mark.parametrize('n,bins,rate', [(300000, 10, 0.8), (300000, 2, 0.8), (100001, 10, 0.5), (1023, 3, 0.9), (1, 2, 0.8)])
